@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — BASELINE.json's metric on its config: rows/sec of join + group-by on the TPC-H Q3 shape at SF100 (config C4).
 
-  python bench.py --gpus N --steps K --warmup W [--impl reference]
+  python bench.py --gpus N --steps K --warmup W [--impl reference] [--dump-outputs DIR]
 
 One step = the whole operator pipeline of the reference's Q3 physical plan (sqllogictest/test_files/tpch/plans/q3.slt.part:60-76)
     FilterExec(c_mktsegment = BUILDING) -> HashJoinExec RightSemi (c_custkey = o_custkey) over FilterExec(o_orderdate < 1995-03-15)
@@ -22,6 +22,9 @@ rows/sec = input rows of the three tables / time.
              reference cannot be built in this image.
 * every timed configuration asserts an order-independent fingerprint of its output at the timed size (a wrong kernel cannot
   produce a number): Q3 vs the CPU arm's fingerprint of the same tables, C2 / C3 vs closed forms over the generators.
+* --dump-outputs DIR : the result rows of the last timed step (l_orderkey, o_orderdate, o_shippriority, revenue) as DIR/<column>.npy,
+             float64, sorted by the group key; above 64 MB a fixed hash sample of the groups (dump_outputs).  The tables come from
+             seeded generators, so two builds run with the same arguments can be compared file for file.
 N > 1 (torchrun): weak scaling — every rank owns an SF100 shard of an SF(100 N) database (see q3_multi_gpu below).
 """
 import argparse
@@ -539,6 +542,39 @@ def secondary_configs(ctx, D, peak):
     return out
 
 
+RESULT_COLUMNS = ("l_orderkey", "o_orderdate", "o_shippriority", "revenue")
+DUMP_MAX_BYTES = 64 << 20
+DUMP_SEED = 0x5EED
+
+
+def dump_outputs(res, out_dir, max_bytes=DUMP_MAX_BYTES):
+    """write the Q3 result rows (the batches a caller of run_q3_fused receives) as out_dir/<column>.npy, float64 (every value here is
+    an integer below 2^53, so the conversion is exact; a NULL would be NaN), rows sorted by the group key.  A result larger than max_bytes
+    keeps the groups whose splitmix64(DUMP_SEED, l_orderkey) % m == 0 for the smallest m that fits: the same groups whatever order the
+    batches came in, so two builds can be compared array for array."""
+    cols = [[] for _ in RESULT_COLUMNS]
+    for b in res:
+        for i, out in enumerate(cols):
+            vals, valid = b.column_numpy(i)
+            vals = vals.astype(np.float64)
+            if valid is not None:
+                vals[~valid] = np.nan
+            out.append(vals)
+    cols = [np.concatenate(c) if c else np.zeros(0, np.float64) for c in cols]
+    order = np.lexsort(cols[2::-1])                         # by l_orderkey, then o_orderdate, o_shippriority
+    cols = [c[order] for c in cols]
+    with np.errstate(over="ignore"):
+        h = splitmix64_np(DUMP_SEED, cols[0].astype(np.uint64))
+    keep, m = np.ones(len(h), bool), 1
+    while keep.sum() * 8 * len(cols) + 128 * len(cols) > max_bytes:       # 128 B: the .npy header of a 1-D array
+        m += 1
+        keep = h % np.uint64(m) == 0
+    os.makedirs(out_dir, exist_ok=True)
+    for name, c in zip(RESULT_COLUMNS, cols):
+        np.save(os.path.join(out_dir, name + ".npy"), c[keep])
+    return int(keep.sum()), m
+
+
 # ---------------------------------------------------------------------------------------------------------------------
 def main():
     ap = argparse.ArgumentParser()
@@ -549,9 +585,14 @@ def main():
     ap.add_argument("--e2e-steps", type=int, default=2)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-secondary", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the result rows of the last timed step as DIR/<column>.npy (float64, at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     rank = int(os.environ.get("RANK", "0")); world = int(os.environ.get("WORLD_SIZE", "1")); local = int(os.environ.get("LOCAL_RANK", "0"))
+    if args.dump_outputs and (args.impl != "ours" or world > 1):
+        ap.error("--dump-outputs writes the single-GPU result of the CUDA path (--impl ours, one process)")
     if args.impl == "reference":
         return run_reference(args, rank, world)
 
@@ -630,6 +671,8 @@ def main():
         fp = Q.result_fingerprint(ctx, last["res"])
         if sf == 100:
             assert fp == Q3_FINGERPRINT_SF100, f"Q3 SF100 fingerprint {fp} != {Q3_FINGERPRINT_SF100}"
+        if args.dump_outputs:
+            dump_outputs(last["res"], args.dump_outputs)
     ms_per_step = ms / args.steps
     in_rows = in_rows_rank * world
     value = in_rows / (ms_per_step / 1000.0)

@@ -4,6 +4,7 @@ from __future__ import annotations
 
 import json
 import os
+import shutil
 from typing import List, Optional, Sequence
 
 import numpy as np
@@ -16,6 +17,12 @@ NP_TYPE = {"int32": np.int32, "int64": np.int64, "uint32": np.uint32, "float64":
 
 def load_golden(name: str):
     return json.load(open(os.path.join(HERE, "golden", name)))
+
+
+def cuda_tool(name: str) -> str:
+    """a CUDA toolkit binary (cuobjdump, ...): from PATH, else from the toolkit the Makefile's nvcc comes from, so the build-evidence
+    tests do not depend on the toolkit's bin/ being on PATH"""
+    return shutil.which(name) or os.path.join("/usr/local/cuda", "bin", name)
 
 
 def col_from_list(values: Sequence, dtype=np.int32):

@@ -7,6 +7,7 @@ import subprocess
 import pytest
 
 from datafusion_b200 import capi
+from harness import cuda_tool
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -29,7 +30,7 @@ def test_library_exports_every_declared_symbol():
 
 
 def test_library_is_sm100a_only():
-    out = subprocess.run(["cuobjdump", "-lelf", capi.LIB_PATH], capture_output=True, text=True).stdout
+    out = subprocess.run([cuda_tool("cuobjdump"), "-lelf", capi.LIB_PATH], capture_output=True, text=True).stdout
     archs = set(re.findall(r"sm_(\d+a?)", out))
     assert archs == {"100a"}, archs
 

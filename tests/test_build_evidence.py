@@ -6,10 +6,11 @@ import re
 import subprocess
 
 from datafusion_b200 import capi
+from harness import cuda_tool
 
 
 def sass(fn):
-    out = subprocess.run(["cuobjdump", "-sass", "-fun", fn, capi.LIB_PATH], capture_output=True, text=True).stdout
+    out = subprocess.run([cuda_tool("cuobjdump"), "-sass", "-fun", fn, capi.LIB_PATH], capture_output=True, text=True).stdout
     return [l for l in out.splitlines() if re.match(r"\s+/\*[0-9a-f]{4,5}\*/", l)]
 
 
